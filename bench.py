@@ -22,6 +22,9 @@ roofline: dominant kernel by CUDA-event share; achieved = algorithmic bytes (SUR
 --impl reference: the CPU restatement of the same plan (oracle/tpch.py q3_cpu: pyarrow Acero, all host cores; no JVM/Spark
           exists in this image) on a bounded sample (the SF10 instance of the same generator).
 --workload q6: the round-1 configuration (BASELINE configs[1], SF10 q6 from Parquet); also reported under `extra` at N=1.
+--dump-outputs DIR: after the timed steps, rank 0 writes the result of the last timed step, one column per file, as
+          DIR/<column>.npy (float64; decimals as their value, dates as days since 1970-01-01).  The inputs are seeded, so two
+          builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -29,6 +32,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -38,7 +42,8 @@ sys.path.insert(0, ROOT)
 
 SF10_ROWS = 59_986_052
 COLS = ["l_shipdate", "l_discount", "l_quantity", "l_extendedprice"]
-CACHE = os.environ.get("B2_BENCH_CACHE", "/tmp/b2_bench_cache")
+# generated Parquet inputs are cached per user: a shared host's temporary directory may hold another user's cache
+CACHE = os.environ.get("B2_BENCH_CACHE", os.path.join(tempfile.gettempdir(), "b2_bench_cache_%d" % os.getuid()))
 NVLINK_GBS = 900.0   # NVLink 5 per direction per GPU (SURVEY §8d exchange roofline)
 Q3_WORKLOAD = "TPC-H SF%g q3 (3 filters, customer JOIN orders JOIN lineitem, group-by (l_orderkey, o_orderdate, o_shippriority), top-10)"
 
@@ -51,6 +56,13 @@ def hbm_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(path, columns):
+    """columns: {name: values} -> path/<name>.npy as float64"""
+    os.makedirs(path, exist_ok=True)
+    for name, vals in columns.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(vals, dtype=np.float64))
 
 
 class ClockSampler:
@@ -233,6 +245,17 @@ def q3_rows_of(table):
     return [(r[0], r[3], r[1], r[2]) for r in table.to_rows()]
 
 
+def q3_columns(rows):
+    """q3 result rows -> output columns (revenue: DECIMAL(36, 4) as its value)"""
+    return {"l_orderkey": [r[0] for r in rows], "revenue": [r[1] / 10**4 for r in rows], "o_orderdate": [r[2] for r in rows],
+            "o_shippriority": [r[3] for r in rows]}
+
+
+def q6_columns(res):
+    """q6 result (unscaled DECIMAL(35, 4) sum, or None) -> output column"""
+    return {"revenue": [np.nan if res is None else res / 10**4]}
+
+
 def q3_host_chunks(sf, rank, world, seed=42):
     """this rank's share of the synthetic tables: {table: [chunk dict]} (numpy, generated on host threads)"""
     from concurrent.futures import ThreadPoolExecutor
@@ -294,6 +317,7 @@ def run_reference(args, rank, world):
         for _ in range(args.steps):
             res = tpch.q6_cpu(raw, cores)
         dt = time.perf_counter() - t0
+        outputs = q6_columns(res)
         rows, name, cfg = args.rows, "tpch_q6_rows_per_sec", {"workload": "TPC-H SF10 q6 (scan+filter+agg), Parquet source (snappy, dictionary, INT64 decimals)", "rows": args.rows, "result": res}
         sample = "full %d-row partition per step; pyarrow %d threads (CPU restatement, NOT Spark)" % (rows, cores)
     else:
@@ -302,19 +326,20 @@ def run_reference(args, rank, world):
         sf = args.ref_sf
         tabs = tpch.q3_arrow_tables(sf, 42, threads=min(32, cores))
         rows = gen.q3_rows(sf)["lineitem"]
-        steps = max(1, min(args.steps, 5))
         for _ in range(min(args.warmup, 1)):
             res = tpch.q3_cpu(*tabs, threads=cores)
         t0 = time.perf_counter()
-        for _ in range(steps):
+        for _ in range(args.steps):
             res = tpch.q3_cpu(*tabs, threads=cores)
         dt = time.perf_counter() - t0
-        args.steps = steps
+        outputs = q3_columns(res)
         name = "tpch_q3_rows_per_sec"
         cfg = {"workload": Q3_WORKLOAD % args.sf, "sf": args.sf, "cpu_plan": "pyarrow Acero on all host cores over the SF%g instance of the same generator (bounded sample)" % sf,
                "sample_sf": sf, "lineitem_rows_per_step": rows, "result_top1": res[0] if res else None}
         sample = "SF%g instance of the synthetic q3 tables (%d lineitem rows) per step, columns cached in host memory; pyarrow Acero on %d threads " \
                  "(CPU restatement, NOT Spark)" % (sf, rows, cores)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     val = rows * args.steps / dt
     line = {"impl": "reference", "metric": name, "value": val, "unit": "rows/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1000 * dt / args.steps, "higher_is_better": True, "scaling": "strong" if args.workload == "q3" else "weak",
@@ -337,9 +362,12 @@ def main():
     ap.add_argument("--cpu-baseline", type=int, default=1)
     ap.add_argument("--extra-q6", type=int, default=1, help="q3 at N=1: also report the SF10 q6 step under `extra`")
     ap.add_argument("--check", type=int, default=1, help="assert the result against the numpy restatement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's result columns to DIR/<column>.npy")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 10 if args.workload == "q3" else 30
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.sf == int(args.sf):
         args.sf = int(args.sf)
     if args.ref_sf == int(args.ref_sf):
@@ -461,6 +489,8 @@ def bench_q3(ctx):
         sampler.start()
     ms, wall, launches, prof, ops, res = timed(True, args.steps, profile=True)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, q3_columns(res))
     xstats0 = comm.stats() if comm else None
     # e2e: pinned host batches -> HostColumnarToGpu inside the timed region
     pinned = []
@@ -700,6 +730,8 @@ def bench_q6(ctx):
         sampler.start()
     ms, wall, launches, prof, res = timed(True, args.steps, profile=True)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, q6_columns(res))
     for _ in range(2):
         step(False)
     ms_e2e, wall_e2e, _, _, res_e2e = timed(False, args.steps)

@@ -1,7 +1,10 @@
 """Generates tests/golden/parquet_testing.json from the Apache parquet-testing corpus that the
 reference vendors under thirdparty/parquet-testing/data (the fixtures its own
-integration_tests/src/main/python/parquet_testing_test.py reads).  Run in the build container
-(where /root/reference exists); the JSON travels to the GPU box, /root/reference does not.
+integration_tests/src/main/python/parquet_testing_test.py reads):
+
+    python tests/golden/make_parquet_golden.py <spark-rapids source checkout>
+
+The tests read only the committed JSON, never the checkout.
 
 Each entry: file bytes (base64), the flat columns we decode, and the expected values as decoded by
 pyarrow (the independent reader), normalised to python values: decimals -> unscaled ints,
@@ -15,7 +18,7 @@ import os
 import pyarrow as pa
 import pyarrow.parquet as pq
 
-SRC = "/root/reference/thirdparty/parquet-testing/data"
+SRC = os.path.join("thirdparty", "parquet-testing", "data")
 FILES = {
     "alltypes_plain.parquet": ["id", "bool_col", "tinyint_col", "smallint_col", "int_col", "bigint_col", "float_col", "double_col", "date_string_col", "string_col"],
     "alltypes_plain.snappy.parquet": ["id", "bool_col", "int_col", "bigint_col", "float_col", "double_col", "string_col"],
@@ -36,7 +39,7 @@ FILES = {
 }
 # the reference's own Scala/pytest fixtures (tests/src/test/resources): Spark-written decimals as INT32/INT64 and as legacy
 # FIXED_LEN_BYTE_ARRAY, timestamp/date columns, a 10-row-group file its split tests read, an unsigned 64-bit column
-SRC2 = "/root/reference/tests/src/test/resources"
+SRC2 = os.path.join("tests", "src", "test", "resources")
 FILES2 = {
     "decimal-test.parquet": ["c_0", "c_1", "c_2", "c_3", "c_4", "c_5"],
     "decimal-test-legacy.parquet": ["c_0", "c_1", "c_2", "c_3", "c_4", "c_5"],
@@ -85,15 +88,15 @@ def norm(v, typ):
     return int(v)
 
 
-def main():
+def main(checkout):
     out = {}
     files = dict(FILES)
     for name in DELTA_FILES:
-        files[name] = delta_int_columns(os.path.join(SRC, name))
-    srcdir = {name: SRC for name in files}
+        files[name] = delta_int_columns(os.path.join(checkout, SRC, name))
+    srcdir = {name: os.path.join(checkout, SRC) for name in files}
     for name, cols in FILES2.items():
         files["spark_rapids_tests/" + name] = cols
-        srcdir["spark_rapids_tests/" + name] = SRC2
+        srcdir["spark_rapids_tests/" + name] = os.path.join(checkout, SRC2)
     for name, cols in files.items():
         path = os.path.join(srcdir[name], os.path.basename(name))
         raw = open(path, "rb").read()
@@ -121,4 +124,5 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    import sys
+    main(sys.argv[1])

@@ -27,7 +27,9 @@ def test_header_cites_reference_for_every_section():
 
 def test_built_for_sm_100a(b2):
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", b2.LIB_PATH], capture_output=True, text=True).stdout
+    from spark_rapids_b200 import build
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")   # the toolkit that built the library; PATH may lack it
+    out = subprocess.run([cuobjdump, "-lelf", b2.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 
