@@ -544,6 +544,16 @@ def _key_of(col, i):
     return v if col.typ[0] == STRING else int(v)
 
 
+def _normalized_key_values(col, rows):
+    """the key values of the given representative rows; floating-point keys come out as +0.0 for -0.0 and the canonical NaN
+    for every NaN, as Spark normalises grouping keys before aggregating (NormalizeFloatingNumbers.scala:29-38)"""
+    vals = col.values[rows]
+    if col.typ[0] in (FLOAT32, FLOAT64):
+        with np.errstate(invalid="ignore"):   # signalling NaN payloads
+            vals = np.where(np.isnan(vals), np.array(np.nan, vals.dtype), vals + np.array(0.0, vals.dtype)).astype(vals.dtype)
+    return vals
+
+
 def groupby_cols(cols, key_idx, specs):
     """AggHelper.performGroupByAggregation: keys then aggregates; group order = first appearance
     (callers compare order-insensitively: output order is unspecified in the reference)"""
@@ -553,8 +563,7 @@ def groupby_cols(cols, key_idx, specs):
         k = tuple(_key_of(cols[c], i) for c in key_idx)
         groups.setdefault(k, []).append(i)
     firsts = [rows[0] for rows in groups.values()]
-    out = [OCol(cols[c].values[firsts], cols[c].valid[firsts], cols[c].typ) if firsts else OCol(cols[c].values[:0], cols[c].valid[:0], cols[c].typ)
-           for c in key_idx]
+    out = [OCol(_normalized_key_values(cols[c], firsts), cols[c].valid[firsts], cols[c].typ) for c in key_idx]
     for spec in specs:
         col = cols[spec[1]] if spec[0] != AGG_COUNT_ALL else None
         vals, oks = [], []

@@ -682,6 +682,17 @@ __global__ void finalize_kernel(GTable gt, const __grid_constant__ AggPlan plan,
   }
 }
 
+// A floating-point group key gathered from the group's representative row may be -0.0 or any NaN payload, whichever row won
+// the slot; the group itself was formed on key_bits.  Writing key_bits back gives +0.0 and the canonical NaN, as Spark's
+// NormalizeFloatingNumbers does before grouping and as the radix regime's packed keys already are.
+__global__ void normalize_float_key_kernel(KeyCol k, int64_t n) {
+  for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x) {
+    const uint64_t b = key_bits(k, r);
+    if (k.width == 4) reinterpret_cast<uint32_t*>(const_cast<void*>(k.data))[r] = (uint32_t)b;
+    else reinterpret_cast<uint64_t*>(const_cast<void*>(k.data))[r] = b;
+  }
+}
+
 // ================================================================================================================================
 // Radix-partitioned group-by for high cardinalities (millions of groups: TPC-H q3's (l_orderkey, o_orderdate, o_shippriority)).
 // The global open-addressing table of the regime above pays several random HBM accesses per row and is sized for the worst
@@ -1375,7 +1386,16 @@ Table* scan_aggregate(const Program* prog, bool has_pred, const Table* t, const 
   std::vector<Column*> result;
   if (nkeys > 0) {
     Table* kt = gather_table(t, rep.as<int32_t>(), ngroups, false, &key_table_cols);
-    for (auto*& c : kt->cols) { result.push_back(c); c = nullptr; }
+    for (auto*& c : kt->cols) {
+      if ((c->dtype == B2_FLOAT32 || c->dtype == B2_FLOAT64) && ngroups > 0) {
+        KeyCol k; memset(&k, 0, sizeof(k));
+        k.data = c->data.p; k.dtype = c->dtype; k.width = dtype_width(c->dtype);
+        normalize_float_key_kernel<<<grid_for(ngroups, 256), 256, 0, stream()>>>(k, ngroups);
+        CUDA_CHECK(cudaGetLastError());
+        count_launch();
+      }
+      result.push_back(c); c = nullptr;
+    }
     kt->cols.clear();
     delete kt;
   }
